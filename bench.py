@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- PESQ + STOI/ESTOI audio-seconds scored per second on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--batch B] [--seconds S]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--batch B] [--seconds S] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[4]): PESQ + STOI/ESTOI of a batch of 8192 x 10 s synthetic
 speech-like pairs at 16 kHz, batch-sharded over the N ranks (strong scaling: 8192 / N items per
@@ -25,6 +25,9 @@ one STOI call over the whole (sharded) batch = 81 920 audio-seconds.
   cpu_baseline / --impl reference: the reference's own CPU path (oracle/_ref: the unmodified reference modules,
            `PESQ(16000, use_gpu=False)` + `STOI(16000, use_gpu=False)` on 64-item chunks) on the host cores, on a
            bounded sample of the same workload; the numpy port (oracle/) beside it / as fallback.
+  --dump-outputs DIR: the score table the last timed step returned, one float32 file per column
+           (DIR/pesq.npy, stoi.npy, estoi.npy, item order).  The inputs are a pure function of the arguments, so two
+           builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -295,6 +298,23 @@ def parity_block(pesq, stoi, clean, deg, gathered, lo, hi, world, device, items)
     return out
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(path: str, table) -> None:
+    """Writes the [batch, 3] score table (PESQ, STOI, ESTOI) as float32 columns.  Above 64 MB in all, a fixed seeded
+    sample of the rows is written instead, with their item indices in items.npy (float64)."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    keep = DUMP_LIMIT_BYTES // (table.shape[1] * 4 + 8)
+    if table.shape[0] > keep:
+        idx = np.sort(np.random.default_rng(0).choice(table.shape[0], keep, replace=False))
+        table = table[idx]
+        np.save(os.path.join(path, "items.npy"), idx.astype(np.float64))
+    for j, name in enumerate(("pesq", "stoi", "estoi")):
+        np.save(os.path.join(path, name + ".npy"), np.ascontiguousarray(table[:, j], dtype=np.float32))
+
+
 # ------------------------------------------------------------------------------------------ main arm
 def main():
     ap = argparse.ArgumentParser()
@@ -309,7 +329,13 @@ def main():
     ap.add_argument("--no-parity", action="store_true")
     ap.add_argument("--no-graph", action="store_true", help="time the direct entry points instead of the CUDA-graph path")
     ap.add_argument("--parity-items", type=int, default=32, help="items per rank scored by the oracle (outside the timed region)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the scores of the last timed step to DIR/{pesq,stoi,estoi}.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the scores of the GPU path; the reference arm keeps none")
     args.warmup = max(args.warmup, 0)
     # stdout carries exactly ONE JSON line (rank 0): anything libraries print there (e.g. NCCL's version banner) is
     # sent to stderr by pointing fd 1 at fd 2 until the line is written
@@ -432,6 +458,8 @@ def main():
     value = audio_s_total / (ms_per_step * 1e-3)
     scores = out.cpu().numpy()
     finite = float(np.isfinite(scores).mean())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, scores)
 
     # ---- parity at this workload, on these tensors (outside the timed region)
     parity = None

@@ -180,3 +180,27 @@ def test_header_is_plain_c_and_a_c_program_can_call_the_library(tmp_path):
     assert rows["version"] == ["200", "200"]
     assert int(rows["null"][0]) == -1 and len(rows["null"]) > 1          # FSEM_E_INVALID + a message
     assert rows["ws"] == ["0"]
+
+
+def test_bench_dump_outputs_writes_float32_columns_and_samples_above_the_limit(tmp_path, monkeypatch):
+    import bench
+    table = np.arange(30, dtype=np.float32).reshape(10, 3)
+    bench.dump_outputs(str(tmp_path / "all"), table)
+    assert sorted(os.listdir(tmp_path / "all")) == ["estoi.npy", "pesq.npy", "stoi.npy"]
+    for j, name in enumerate(("pesq", "stoi", "estoi")):
+        col = np.load(tmp_path / "all" / (name + ".npy"))
+        assert col.dtype == np.float32 and np.array_equal(col, table[:, j])
+    monkeypatch.setattr(bench, "DUMP_LIMIT_BYTES", 4 * (3 * 4 + 8))      # room for 4 rows and their indices
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), table)
+    idx = np.load(tmp_path / "a" / "items.npy")
+    assert idx.dtype == np.float64 and len(idx) == 4 and np.array_equal(idx, np.load(tmp_path / "b" / "items.npy"))
+    assert np.array_equal(np.load(tmp_path / "a" / "stoi.npy"), table[idx.astype(int), 1])
+    assert sum(f.stat().st_size - 128 for f in (tmp_path / "a").iterdir()) <= bench.DUMP_LIMIT_BYTES   # 128: .npy header
+
+
+def test_bench_rejects_zero_timed_steps():
+    import subprocess
+    import sys
+    res = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"], capture_output=True, text=True)
+    assert res.returncode == 2 and "--steps must be at least 1" in res.stderr
