@@ -11,7 +11,7 @@ import ctypes as C
 import torch
 
 from . import _lib
-from .base import BaseMetric
+from .base import BaseMetric, check_score, make_batch, score_host, stream_ptr
 from .design import pesq_design
 
 
@@ -47,42 +47,20 @@ class PESQ(BaseMetric):
         lens = self._lengths_tensor(lengths, b, n, clean.device)
         mos = torch.empty(b, dtype=torch.float32, device=clean.device)
         status = torch.empty(b, dtype=torch.int32, device=clean.device)
+        batch, clean, deg = make_batch(clean, deg, lens)
         with torch.cuda.device(clean.device):
-            ws_bytes = self._lib.fsem_pesq_workspace_bytes(self._ctx, b, n)
-            ws = self._get_workspace(ws_bytes)
-            batch = _lib.Batch(clean.data_ptr(), deg.data_ptr(), lens.data_ptr() if lens is not None else None,
-                               b, n, clean.stride(0) if b > 1 else max(n, clean.stride(0)))
-            if deg.stride(0) != clean.stride(0) and b > 1:
-                deg = deg.contiguous(); clean = clean.contiguous()
-                batch.clean, batch.deg, batch.stride = clean.data_ptr(), deg.data_ptr(), n
-            self._check_score(self._lib.fsem_pesq_score(
+            ws = self._get_workspace(self._lib.fsem_pesq_workspace_bytes(self._ctx, b, n))
+            check_score(self._lib.fsem_pesq_score(
                 self._ctx, C.byref(batch), _lib.dtype_code(clean.dtype), mos.data_ptr(), status.data_ptr(), ws.data_ptr(),
-                ws.numel(), C.c_void_p(torch.cuda.current_stream(clean.device).cuda_stream)))
+                ws.numel(), stream_ptr(clean.device)))
         self._last_shape = (b, n)
         return mos, status
 
     def score_host(self, clean: torch.Tensor, deg: torch.Tensor, lengths=None):
         """Host-resident scoring: CPU [B, n] float32 / int16 / float16 tensors in, CPU tensors out; the
         library overlaps the host->device copies with compute."""
-        b, n = clean.shape
-        lens = self._lengths_tensor(lengths, b, n, "cpu")
-        mos = torch.empty(b, dtype=torch.float32)
-        status = torch.empty(b, dtype=torch.int32)
-        if clean.stride(0) != deg.stride(0) and b > 1:
-            clean, deg = clean.contiguous(), deg.contiguous()
-        with torch.cuda.device(self.device):
-            self._check_score(self._lib.fsem_score_host(
-                self._ctx, None, clean.data_ptr(), deg.data_ptr(), _lib.dtype_code(clean.dtype),
-                lens.data_ptr() if lens is not None else None, b, n, clean.stride(0) if b > 1 else n,
-                mos.data_ptr(), status.data_ptr(), None, None, None, None))
+        mos, status, _, _, _ = score_host(self, None, clean, deg, lengths)
         return mos, status
-
-    @staticmethod
-    def _check_score(code: int):
-        if code == _lib.FSEM_E_TOO_SHORT:
-            # the reference's unfold(1, size=20, step=10) fails the same way (PESQ.py:169)
-            raise RuntimeError(_lib.load().fsem_last_error().decode())
-        _lib.check(code)
 
     def compute_metric(self, clean_speech, denoised_speech, lengths=None) -> list[dict[str, float]]:
         assert clean_speech is not None                                   # PESQ.py:235
@@ -103,7 +81,7 @@ class PESQ(BaseMetric):
         b, n = self._last_shape
         frames = C.c_int64()
         with torch.cuda.device(self.device):
-            stream = C.c_void_p(torch.cuda.current_stream().cuda_stream)
+            stream = stream_ptr(self.device)
             _lib.check(self._lib.fsem_pesq_debug_taps(self._ctx, b, n, self._workspace.data_ptr(), None, None,
                                                       C.byref(frames), stream))
             bark = torch.empty(2, b, frames.value, 49, dtype=torch.float32, device=self.device)

@@ -8,7 +8,7 @@ import ctypes as C
 import torch
 
 from . import _lib
-from .base import BaseMetric
+from .base import BaseMetric, make_batch, stream_ptr
 
 
 class SDR(BaseMetric):
@@ -31,14 +31,11 @@ class SDR(BaseMetric):
         clean, deg, lens = self._resample_pair(clean, deg, lens)             # base.py:19-20
         b, n = clean.shape
         out = torch.empty(b, dtype=torch.float32, device=clean.device)
+        batch, clean, deg = make_batch(clean, deg, lens)
         with torch.cuda.device(clean.device):
             ws = self._get_workspace(self._lib.fsem_sdr_workspace_bytes(b, n))
-            if deg.stride(0) != clean.stride(0) and b > 1:
-                deg = deg.contiguous(); clean = clean.contiguous()
-            batch = _lib.Batch(clean.data_ptr(), deg.data_ptr(), lens.data_ptr() if lens is not None else None,
-                               b, n, clean.stride(0) if b > 1 else max(n, clean.stride(0)))
             _lib.check(self._lib.fsem_sdr_score_f32(C.byref(batch), out.data_ptr(), ws.data_ptr(), ws.numel(),
-                                                    C.c_void_p(torch.cuda.current_stream(clean.device).cuda_stream)))
+                                                    stream_ptr(clean.device)))
         return out
 
     def compute_metric(self, clean_speech, denoised_speech, lengths=None) -> list[dict[str, float]]:

@@ -12,7 +12,7 @@ import warnings
 import torch
 
 from . import _lib
-from .base import BaseMetric
+from .base import BaseMetric, make_batch, score_host, stream_ptr
 from .design import stoi_design
 
 
@@ -48,17 +48,12 @@ class STOI(BaseMetric):
         scores = torch.empty(2, b, dtype=torch.float32, device=clean.device)
         kept = torch.empty(b, dtype=torch.int32, device=clean.device)
         status = torch.empty(b, dtype=torch.int32, device=clean.device)
+        batch, clean, deg = make_batch(clean, deg, lens)
         with torch.cuda.device(clean.device):
-            ws_bytes = self._lib.fsem_stoi_workspace_bytes(self._ctx, b, n)
-            ws = self._get_workspace(ws_bytes)
-            if deg.stride(0) != clean.stride(0) and b > 1:
-                deg = deg.contiguous(); clean = clean.contiguous()
-            batch = _lib.Batch(clean.data_ptr(), deg.data_ptr(), lens.data_ptr() if lens is not None else None,
-                               b, n, clean.stride(0) if b > 1 else max(n, clean.stride(0)))
+            ws = self._get_workspace(self._lib.fsem_stoi_workspace_bytes(self._ctx, b, n))
             _lib.check(self._lib.fsem_stoi_score(
                 self._ctx, C.byref(batch), _lib.dtype_code(clean.dtype), scores[0].data_ptr(), scores[1].data_ptr(), kept.data_ptr(),
-                status.data_ptr(), ws.data_ptr(), ws.numel(),
-                C.c_void_p(torch.cuda.current_stream(clean.device).cuda_stream)))
+                status.data_ptr(), ws.data_ptr(), ws.numel(), stream_ptr(clean.device)))
         self._last_shape = (b, n)
         self._last_lengths = lens
         return scores, kept, status
@@ -74,23 +69,12 @@ class STOI(BaseMetric):
         with torch.cuda.device(self.device):
             _lib.check(self._lib.fsem_stoi_mask_margin(
                 self._ctx, b, n, lens.data_ptr() if lens is not None else None, self._workspace.data_ptr(),
-                out.data_ptr(), C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)))
+                out.data_ptr(), stream_ptr(self.device)))
         return out
 
     def score_host(self, clean: torch.Tensor, deg: torch.Tensor, lengths=None):
         """Host-resident scoring: CPU [B, n] float32 / int16 / float16 tensors in, CPU tensors out."""
-        b, n = clean.shape
-        lens = self._lengths_tensor(lengths, b, n, "cpu")
-        scores = torch.empty(2, b, dtype=torch.float32)
-        kept = torch.empty(b, dtype=torch.int32)
-        status = torch.empty(b, dtype=torch.int32)
-        if clean.stride(0) != deg.stride(0) and b > 1:
-            clean, deg = clean.contiguous(), deg.contiguous()
-        with torch.cuda.device(self.device):
-            _lib.check(self._lib.fsem_score_host(
-                None, self._ctx, clean.data_ptr(), deg.data_ptr(), _lib.dtype_code(clean.dtype),
-                lens.data_ptr() if lens is not None else None, b, n, clean.stride(0) if b > 1 else n,
-                None, None, scores[0].data_ptr(), scores[1].data_ptr(), kept.data_ptr(), status.data_ptr()))
+        _, _, scores, kept, status = score_host(None, self, clean, deg, lengths)
         return scores, kept, status
 
     def compute_metric(self, clean_speech, denoised_speech, lengths=None) -> list[dict[str, float]]:
@@ -116,7 +100,7 @@ class STOI(BaseMetric):
         b, n = self._last_shape
         dims = (C.c_int64 * 3)()
         with torch.cuda.device(self.device):
-            stream = C.c_void_p(torch.cuda.current_stream().cuda_stream)
+            stream = stream_ptr(self.device)
             ws = self._workspace.data_ptr()
             _lib.check(self._lib.fsem_stoi_debug_taps(self._ctx, b, n, ws, None, None, None, dims, stream))
             mask = torch.empty(b, dims[0], dtype=torch.int32, device=self.device)

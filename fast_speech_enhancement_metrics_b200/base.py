@@ -28,6 +28,58 @@ import torch
 from . import _lib
 
 
+def stream_ptr(device) -> C.c_void_p:
+    """The current CUDA stream of `device` as the library's `void* stream` argument."""
+    return C.c_void_p(torch.cuda.current_stream(device).cuda_stream)
+
+
+def _ptr(t):
+    return t.data_ptr() if t is not None else None
+
+
+def make_batch(clean: torch.Tensor, deg: torch.Tensor, lens):
+    """[B, n] clean / deg rows and optional int32 lengths[B] -> (_lib.Batch, clean, deg).  The library takes one row
+    pitch for both signals, so rows of different pitch are made contiguous; the returned tensors are the ones the
+    struct points at and must stay alive for the call."""
+    b, n = clean.shape
+    if deg.stride(0) != clean.stride(0) and b > 1:
+        clean, deg = clean.contiguous(), deg.contiguous()
+    batch = _lib.Batch(clean.data_ptr(), deg.data_ptr(), _ptr(lens), b, n,
+                       clean.stride(0) if b > 1 else max(n, clean.stride(0)))
+    return batch, clean, deg
+
+
+def check_score(code: int) -> None:
+    if code == _lib.FSEM_E_TOO_SHORT:
+        # the reference's unfold(1, size=20, step=10) fails the same way (PESQ.py:169)
+        raise RuntimeError(_lib.load().fsem_last_error().decode())
+    _lib.check(code)
+
+
+def score_host(pesq, stoi, clean: torch.Tensor, deg: torch.Tensor, lengths=None):
+    """Host-resident scoring of PESQ, STOI or both on one upload (fsem_score_host): CPU [B, n] float32 / int16 /
+    float16 rows in, CPU tensors out: (mos[B], pesq_status[B], scores[2, B] = STOI / ESTOI rows, kept[B],
+    stoi_status[B]), None for the outputs of a metric that is None.  The library overlaps the host->device copies
+    with compute."""
+    owner = pesq if pesq is not None else stoi
+    b, n = clean.shape
+    lens = BaseMetric._lengths_tensor(lengths, b, n, "cpu")
+    batch, clean, deg = make_batch(clean, deg, lens)
+    mos = pst = scores = kept = sst = None
+    if pesq is not None:
+        mos, pst = torch.empty(b, dtype=torch.float32), torch.empty(b, dtype=torch.int32)
+    if stoi is not None:
+        scores = torch.empty(2, b, dtype=torch.float32)
+        kept, sst = torch.empty(b, dtype=torch.int32), torch.empty(b, dtype=torch.int32)
+    with torch.cuda.device(owner.device):
+        check_score(owner._lib.fsem_score_host(
+            pesq._ctx if pesq is not None else None, stoi._ctx if stoi is not None else None, batch.clean, batch.deg,
+            _lib.dtype_code(clean.dtype), batch.lengths, b, n, batch.stride, _ptr(mos), _ptr(pst),
+            _ptr(None if scores is None else scores[0]), _ptr(None if scores is None else scores[1]), _ptr(kept),
+            _ptr(sst)))
+    return mos, pst, scores, kept, sst
+
+
 class BaseMetric(ABC):
     higher_is_better: bool
     EXPECTED_SAMPLING_RATE: int
@@ -78,8 +130,7 @@ class BaseMetric(ABC):
             with torch.cuda.device(audio.device):
                 _lib.check(self._lib.fsem_ingest_f32(
                     audio.data_ptr(), code, b, n, audio.stride(0) if b > 1 else max(n, audio.stride(0)),
-                    out.data_ptr(), out.stride(0),
-                    C.c_void_p(torch.cuda.current_stream(audio.device).cuda_stream)))
+                    out.data_ptr(), out.stride(0), stream_ptr(audio.device)))
         return out
 
     def prepare_inputs(self, clean_speech, denoised_speech):
@@ -136,15 +187,10 @@ class BaseMetric(ABC):
         pitch = (L + 3) // 4 * 4
         out = torch.empty(2, b, pitch, dtype=torch.float32, device=self.device)
         new_lens = torch.empty(b, dtype=torch.int32, device=self.device) if lens is not None else None
+        batch, clean, deg = make_batch(clean, deg, lens)
         with torch.cuda.device(self.device):
-            if deg.stride(0) != clean.stride(0) and b > 1:
-                deg = deg.contiguous(); clean = clean.contiguous()
-            batch = _lib.Batch(clean.data_ptr(), deg.data_ptr(), lens.data_ptr() if lens is not None else None,
-                               b, n, clean.stride(0) if b > 1 else max(n, clean.stride(0)))
-            _lib.check(self._lib.fsem_resample_f32(
-                self._resampler, C.byref(batch), out.data_ptr(), pitch,
-                new_lens.data_ptr() if new_lens is not None else None,
-                C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)))
+            _lib.check(self._lib.fsem_resample_f32(self._resampler, C.byref(batch), out.data_ptr(), pitch, _ptr(new_lens),
+                                                   stream_ptr(self.device)))
         return out[0, :, :L], out[1, :, :L], new_lens
 
     def _score_host_overlapped(self, clean: torch.Tensor, deg: torch.Tensor, lengths=None) -> torch.Tensor:

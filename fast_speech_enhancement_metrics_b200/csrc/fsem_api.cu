@@ -5,6 +5,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <memory>
 #include <new>
 #include <vector>
 
@@ -113,6 +114,21 @@ struct HostPipe {
     void* out = nullptr;                  // device score columns for the WHOLE batch (one D2H at the end)
     size_t out_bytes = 0;
 
+    HostPipe() = default;
+    HostPipe(const HostPipe&) = delete;
+    HostPipe& operator=(const HostPipe&) = delete;
+    ~HostPipe() {
+        for (int i = 0; i < 2; ++i) {
+            if (in[i]) cudaFree(in[i]);
+            if (copied[i]) cudaEventDestroy(copied[i]);
+            if (done[i]) cudaEventDestroy(done[i]);
+        }
+        if (ws) cudaFree(ws);
+        if (out) cudaFree(out);
+        if (copy) cudaStreamDestroy(copy);
+        if (compute) cudaStreamDestroy(compute);
+    }
+
     int init() {
         if (copy) return FSEM_OK;
         FSEM_CUDA(cudaStreamCreateWithFlags(&copy, cudaStreamNonBlocking));
@@ -145,17 +161,6 @@ struct HostPipe {
             out_bytes = out_b;
         }
         return FSEM_OK;
-    }
-    void destroy() {
-        for (int i = 0; i < 2; ++i) {
-            if (in[i]) cudaFree(in[i]);
-            if (copied[i]) cudaEventDestroy(copied[i]);
-            if (done[i]) cudaEventDestroy(done[i]);
-        }
-        if (ws) cudaFree(ws);
-        if (out) cudaFree(out);
-        if (copy) cudaStreamDestroy(copy);
-        if (compute) cudaStreamDestroy(compute);
     }
 };
 
@@ -191,6 +196,75 @@ int dispatch_dtype(int dtype, F&& fn) {
     }
 }
 
+// Checks of a batch of (clean, deg) row pairs, in the one order every entry point uses.  Returns FSEM_E_INVALID (the
+// message names `who`), kEmptyBatch for a valid empty batch, or FSEM_OK.  [n_min, n_max]: the signal lengths the entry
+// point takes.  With `n_checked_when_empty` an empty batch needs a valid n too (LSD, SDR, the resampler); otherwise an
+// empty batch is accepted whatever its n (PESQ, STOI, the host pipeline).
+constexpr int kEmptyBatch = 1;
+constexpr int64_t kMaxN = (int64_t(1) << 30) - 1;      // sample indices of the device kernels stay below 2^30
+int check_batch(const char* who, const void* clean, const void* deg, int64_t batch, int64_t n, int64_t stride,
+                int64_t n_min, int64_t n_max, bool n_checked_when_empty) {
+    const bool n_ok = n >= n_min && n <= n_max;
+    if (batch < 0 || n < 0 || stride < n || (n_checked_when_empty && !n_ok))
+        return fail(FSEM_E_INVALID, "%s: bad shape batch=%lld n=%lld stride=%lld", who, (long long)batch, (long long)n,
+                    (long long)stride);
+    if (batch == 0) return kEmptyBatch;
+    if (!clean || !deg) return fail(FSEM_E_INVALID, "%s: null input", who);
+    if (!n_ok)
+        return fail(FSEM_E_INVALID, "%s: n=%lld outside [%lld, %lld]", who, (long long)n, (long long)n_min,
+                    (long long)n_max);
+    return FSEM_OK;
+}
+
+// The general polyphase resampler (stoi_resample_kernel): rates divided by their gcd, kernel half-width, the taps
+// [neu][ntaps] and their device copy.  PESQ's resample-on-ingest, STOI's general path and fsem_resampler_t use it.
+struct Resampler {
+    int orig = 1, neu = 1, width = 0, ntaps = 0;
+    float* d_taps = nullptr;
+
+    Resampler() = default;
+    Resampler(const Resampler&) = delete;
+    Resampler& operator=(const Resampler&) = delete;
+    ~Resampler() { if (d_taps) cudaFree(d_taps); }
+
+    // the design rule of the kernel; makes no CUDA call
+    static int check(const char* who, int orig, int neu, int width, int ntaps, const float* taps) {
+        if (orig <= 0 || neu <= 0 || width < 0 || !taps || ntaps != 2 * width + orig)
+            return fail(FSEM_E_INVALID, "%s: bad resampling kernel (ntaps must be 2*width+orig)", who);
+        return FSEM_OK;
+    }
+    // keeps a design that passed check() and copies its taps to the device
+    int upload(int orig_, int neu_, int width_, int ntaps_, const float* taps) {
+        orig = orig_; neu = neu_; width = width_; ntaps = ntaps_;
+        FSEM_CUDA(cudaMalloc(&d_taps, sizeof(float) * neu * ntaps));
+        FSEM_CUDA(cudaMemcpy(d_taps, taps, sizeof(float) * neu * ntaps, cudaMemcpyHostToDevice));
+        return FSEM_OK;
+    }
+    // clean and deg rows of `dtype` -> fp32 rows [2, batch, out_stride] (clean rows, then deg rows); with per-item
+    // lengths and a non-null `lengths_out`, also the resampled lengths
+    int launch(const char* who, KernelId id, const fsem_batch_t* in, int dtype, float* out, int64_t out_stride,
+               int32_t* lengths_out, cudaStream_t stream) const {
+        const int64_t bps = ceil_div(stoi_resampled_len(in->n, orig, neu), 256);
+        if (bps * 2 * in->batch >= (int64_t(1) << 31))
+            return fail(FSEM_E_INVALID, "%s: batch x samples too large for one launch; split the batch", who);
+        { ProfScope prof_(id, stream);
+          dispatch_dtype(dtype, [&](auto tag) {
+              using T = decltype(tag);
+              stoi_resample_kernel<T><<<(unsigned)(bps * 2 * in->batch), 256, 0, stream>>>(
+                  reinterpret_cast<const T*>(in->clean), reinterpret_cast<const T*>(in->deg), in->lengths, in->batch,
+                  in->n, in->stride, d_taps, orig, neu, width, ntaps, out, out_stride, (int)bps);
+              return FSEM_OK;
+          }); }
+        FSEM_LAUNCHED();
+        if (in->lengths && lengths_out) {
+            resampled_lengths_kernel<<<(unsigned)ceil_div(in->batch, 256), 256, 0, stream>>>(
+                in->lengths, in->batch, in->n, orig, neu, lengths_out);
+            FSEM_LAUNCHED();
+        }
+        return FSEM_OK;
+    }
+};
+
 }  // namespace
 
 // ------------------------------------------------------------------------------------------------
@@ -220,8 +294,7 @@ struct fsem_pesq_ctx {
     PesqFilterCoef coef;
     int warm = 640;
     PesqTables* d_tab = nullptr;
-    int rs_orig = 1, rs_neu = 1, rs_width = 0, rs_ntaps = 0;   // resample-on-ingest to 16 kHz (base.py:19-20)
-    float* d_rs_taps = nullptr;
+    Resampler rs;                    // resample-on-ingest to 16 kHz (base.py:19-20); 1:1 when the input is 16 kHz
     int spec_ctas_per_sm = 2;
     int filt_ctas_per_sm = 4;
     // > 0: plan the IIR time-chunk grid as for a batch of this size (fsem_graph_create scores a batch in slices and
@@ -229,6 +302,8 @@ struct fsem_pesq_ctx {
     // and unsliced scoring agree bit for bit)
     int64_t plan_batch_hint = 0;
     HostPipe pipe;
+
+    ~fsem_pesq_ctx() { if (d_tab) cudaFree(d_tab); }
 };
 
 namespace {
@@ -247,8 +322,8 @@ PesqPlan pesq_plan(const fsem_pesq_ctx* ctx, int64_t batch, int64_t n_in) {
     PesqPlan p{};
     p.batch = batch;
     p.n_in = n_in;
-    p.resample = ctx->rs_orig != ctx->rs_neu;
-    const int64_t n = stoi_resampled_len(n_in, ctx->rs_orig, ctx->rs_neu);
+    p.resample = ctx->rs.orig != ctx->rs.neu;
+    const int64_t n = stoi_resampled_len(n_in, ctx->rs.orig, ctx->rs.neu);
     p.rstride = round_up(n > 0 ? n : 1, 4);
     p.n = n;
     // the spectrum kernel fetches whole 1 KB half-frames with bulk copies: the last frame ends at most 255 samples
@@ -302,24 +377,10 @@ PesqPlan pesq_plan(const fsem_pesq_ctx* ctx, int64_t batch, int64_t n_in) {
 extern "C" int fsem_pesq_create(fsem_pesq_ctx_t** out, const fsem_pesq_design_t* d) {
     if (!out || !d) return fail(FSEM_E_INVALID, "fsem_pesq_create: null argument");
     *out = nullptr;
-    fsem_pesq_ctx* ctx = new (std::nothrow) fsem_pesq_ctx();
-    if (!ctx) return fail(FSEM_E_INVALID, "out of host memory");
-    int rc = query_device(ctx->dev);
-    if (rc != FSEM_OK) { delete ctx; return rc; }
-    ctx->coef.k = d->bp_direct;
-    for (int s = 0; s < FSEM_BP_SECTIONS; ++s) {
-        ctx->coef.c0[s] = d->bp_c0[s]; ctx->coef.c1[s] = d->bp_c1[s];
-        ctx->coef.a1[s] = d->bp_a1[s]; ctx->coef.a2[s] = d->bp_a2[s];
-    }
-    ctx->coef.pb0 = d->pre_b[0]; ctx->coef.pb1 = d->pre_b[1]; ctx->coef.pb2 = d->pre_b[2];
-    ctx->coef.pa1 = d->pre_a[0]; ctx->coef.pa2 = d->pre_a[1];
-    ctx->warm = (int)round_up(d->warmup > 0 ? d->warmup : 640, 32);
-    for (int k = 0; k < 15; ++k) {
-        if (fabsf(d->taper[k] - (float)(k + 1) * 0.0625f) > 1e-7f) {
-            delete ctx;
+    // the whole design is checked before the first CUDA call
+    for (int k = 0; k < 15; ++k)
+        if (fabsf(d->taper[k] - (float)(k + 1) * 0.0625f) > 1e-7f)
             return fail(FSEM_E_INVALID, "fsem_pesq_create: taper must be k/16 (PESQ.py:90)");
-        }
-    }
     PesqTables h{};
     memcpy(h.hann, d->hann, sizeof(h.hann));
     double wtot = 0.0;
@@ -328,16 +389,12 @@ extern "C" int fsem_pesq_create(fsem_pesq_ctx_t** out, const fsem_pesq_design_t*
         h.band_count[b] = d->band_num_bins[b];
         const int expect_first = b == 0 ? 0 : h.band_first[b - 1] + h.band_count[b - 1];
         if (h.band_first[b] != expect_first || h.band_count[b] < 1 || h.band_count[b] > 32 ||
-            h.band_first[b] + h.band_count[b] > 256) {
-            delete ctx;
+            h.band_first[b] + h.band_count[b] > 256)
             return fail(FSEM_E_INVALID, "fsem_pesq_create: Bark bands must tile bins 0..255 contiguously, at most 32 bins each (band %d)", b);
-        }
         {   // the spectrum kernel gathers a band from at most 1 (bands 0..31) / 4 (bands 32..48) earlier 8-bin groups
             const int span = ((h.band_first[b] + h.band_count[b] - 1) >> 3) - (h.band_first[b] >> 3);
-            if (span > (b < 32 ? kBarkPiecesLow : kBarkPiecesHigh)) {
-                delete ctx;
+            if (span > (b < 32 ? kBarkPiecesLow : kBarkPiecesHigh))
                 return fail(FSEM_E_INVALID, "fsem_pesq_create: Bark band %d spans %d groups of 8 bins (unsupported layout)", b, span + 1);
-            }
         }
         h.pow_dens[b] = d->pow_dens[b];
         h.thresh[b] = d->thresh[b];
@@ -347,58 +404,43 @@ extern "C" int fsem_pesq_create(fsem_pesq_ctx_t** out, const fsem_pesq_design_t*
         if (b >= 1) wtot += (double)d->width_bark[b];
     }
     h.width_total = (float)wtot;
-    cudaError_t e = cudaMalloc(&ctx->d_tab, sizeof(PesqTables));
-    if (e == cudaSuccess) e = cudaMemcpy(ctx->d_tab, &h, sizeof(h), cudaMemcpyHostToDevice);
-    if (e != cudaSuccess) {
-        if (ctx->d_tab) cudaFree(ctx->d_tab);
-        delete ctx;
-        return fail(FSEM_E_CUDA, "fsem_pesq_create: %s", cudaGetErrorString(e));
+    const bool resample = d->rs_orig != d->rs_neu;
+    int rc = resample ? Resampler::check("fsem_pesq_create", d->rs_orig, d->rs_neu, d->rs_width, d->rs_ntaps, d->rs_taps)
+                      : FSEM_OK;
+    if (rc != FSEM_OK) return rc;
+
+    std::unique_ptr<fsem_pesq_ctx> ctx(new (std::nothrow) fsem_pesq_ctx());
+    if (!ctx) return fail(FSEM_E_INVALID, "out of host memory");
+    ctx->coef.k = d->bp_direct;
+    for (int s = 0; s < FSEM_BP_SECTIONS; ++s) {
+        ctx->coef.c0[s] = d->bp_c0[s]; ctx->coef.c1[s] = d->bp_c1[s];
+        ctx->coef.a1[s] = d->bp_a1[s]; ctx->coef.a2[s] = d->bp_a2[s];
     }
-    if (e == cudaSuccess && d->rs_orig != d->rs_neu) {
-        if (d->rs_orig <= 0 || d->rs_neu <= 0 || !d->rs_taps || d->rs_ntaps != 2 * d->rs_width + d->rs_orig) {
-            cudaFree(ctx->d_tab);
-            delete ctx;
-            return fail(FSEM_E_INVALID, "fsem_pesq_create: bad resampling kernel (ntaps must be 2*width+orig)");
-        }
-        ctx->rs_orig = d->rs_orig; ctx->rs_neu = d->rs_neu; ctx->rs_width = d->rs_width; ctx->rs_ntaps = d->rs_ntaps;
-        e = cudaMalloc(&ctx->d_rs_taps, sizeof(float) * d->rs_neu * d->rs_ntaps);
-        if (e == cudaSuccess)
-            e = cudaMemcpy(ctx->d_rs_taps, d->rs_taps, sizeof(float) * d->rs_neu * d->rs_ntaps, cudaMemcpyHostToDevice);
-        if (e != cudaSuccess) {
-            cudaFree(ctx->d_tab);
-            if (ctx->d_rs_taps) cudaFree(ctx->d_rs_taps);
-            delete ctx;
-            return fail(FSEM_E_CUDA, "fsem_pesq_create: %s", cudaGetErrorString(e));
-        }
-    }
-    e = cudaFuncSetAttribute(pesq_spectrum_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSpecDynSmem);
-    if (e == cudaSuccess)
-        e = cudaFuncSetAttribute(pesq_bark_kernel<kBarkThreadsWide, kBarkTileWide>,
-                                 cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bark_dyn_smem(kBarkTileWide));
-    if (e == cudaSuccess && bark_dyn_smem(kBarkTile) > 0)
-        e = cudaFuncSetAttribute(pesq_bark_kernel<kBarkThreads, kBarkTile>,
-                                 cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bark_dyn_smem(kBarkTile));
-    if (e != cudaSuccess) {
-        cudaFree(ctx->d_tab);
-        if (ctx->d_rs_taps) cudaFree(ctx->d_rs_taps);
-        delete ctx;
-        return fail(FSEM_E_CUDA, "fsem_pesq_create: %s", cudaGetErrorString(e));
-    }
+    ctx->coef.pb0 = d->pre_b[0]; ctx->coef.pb1 = d->pre_b[1]; ctx->coef.pb2 = d->pre_b[2];
+    ctx->coef.pa1 = d->pre_a[0]; ctx->coef.pa2 = d->pre_a[1];
+    ctx->warm = (int)round_up(d->warmup > 0 ? d->warmup : 640, 32);
+    if ((rc = query_device(ctx->dev)) != FSEM_OK) return rc;
+    FSEM_CUDA(cudaMalloc(&ctx->d_tab, sizeof(PesqTables)));
+    FSEM_CUDA(cudaMemcpy(ctx->d_tab, &h, sizeof(h), cudaMemcpyHostToDevice));
+    if (resample && (rc = ctx->rs.upload(d->rs_orig, d->rs_neu, d->rs_width, d->rs_ntaps, d->rs_taps)) != FSEM_OK)
+        return rc;
+    FSEM_CUDA(cudaFuncSetAttribute(pesq_spectrum_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSpecDynSmem));
+    FSEM_CUDA(cudaFuncSetAttribute(pesq_bark_kernel<kBarkThreadsWide, kBarkTileWide>,
+                                   cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bark_dyn_smem(kBarkTileWide)));
+    if (bark_dyn_smem(kBarkTile) > 0)
+        FSEM_CUDA(cudaFuncSetAttribute(pesq_bark_kernel<kBarkThreads, kBarkTile>,
+                                       cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bark_dyn_smem(kBarkTile)));
     int occ = 0;
     if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, pesq_spectrum_kernel, kSpecWarps * 32, kSpecDynSmem) == cudaSuccess && occ > 0)
         ctx->spec_ctas_per_sm = occ;
     occ = 0;
     if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, pesq_filter_tiled_kernel<false, float>, kFiltWarps * 32, 0) == cudaSuccess && occ > 0)
         ctx->filt_ctas_per_sm = occ;
-    *out = ctx;
+    *out = ctx.release();
     return FSEM_OK;
 }
 
 extern "C" int fsem_pesq_destroy(fsem_pesq_ctx_t* ctx) {
-    if (!ctx) return FSEM_OK;
-    ctx->pipe.destroy();
-    if (ctx->d_tab) cudaFree(ctx->d_tab);
-    if (ctx->d_rs_taps) cudaFree(ctx->d_rs_taps);
     delete ctx;
     return FSEM_OK;
 }
@@ -418,15 +460,10 @@ extern "C" int fsem_pesq_score_f32(fsem_pesq_ctx_t* ctx, const fsem_batch_t* in,
 // as they are; `in->clean` / `in->deg` point at rows of `dtype`, `in->stride` counts elements.
 extern "C" int fsem_pesq_score(fsem_pesq_ctx_t* ctx, const fsem_batch_t* in, int dtype, float* mos_out,
                                int32_t* status_out, void* workspace, size_t workspace_bytes, void* stream_v) {
-    if (!ctx || !in || !mos_out) return fail(FSEM_E_INVALID, "fsem_pesq_score_f32: null argument");
-    const size_t es = dtype_size(dtype);
-    if (es == 0) return fail(FSEM_E_INVALID, "fsem_pesq_score: unknown dtype %d", dtype);
-    if (in->batch < 0 || in->n < 0 || in->stride < in->n)
-        return fail(FSEM_E_INVALID, "fsem_pesq_score_f32: bad shape batch=%lld n=%lld stride=%lld",
-                    (long long)in->batch, (long long)in->n, (long long)in->stride);
-    if (in->batch == 0) return FSEM_OK;
-    if (!in->clean || !in->deg) return fail(FSEM_E_INVALID, "fsem_pesq_score_f32: null input");
-    if (in->n >= (int64_t(1) << 30)) return fail(FSEM_E_INVALID, "fsem_pesq_score_f32: n too large");
+    if (!ctx || !in || !mos_out) return fail(FSEM_E_INVALID, "fsem_pesq_score: null argument");
+    if (dtype_size(dtype) == 0) return fail(FSEM_E_INVALID, "fsem_pesq_score: unknown dtype %d", dtype);
+    if (int rc = check_batch("fsem_pesq_score", in->clean, in->deg, in->batch, in->n, in->stride, 0, kMaxN, false))
+        return rc == kEmptyBatch ? FSEM_OK : rc;
     const PesqPlan p = pesq_plan(ctx, in->batch, in->n);
     // without per-item lengths every item has n samples: fewer than 20 frames is the reference's
     // RuntimeError from unfold (PESQ.py:169)
@@ -434,7 +471,7 @@ extern "C" int fsem_pesq_score(fsem_pesq_ctx_t* ctx, const fsem_batch_t* in, int
         return fail(FSEM_E_TOO_SHORT, "PESQ needs at least 20 frames of 512/256 samples at 16 kHz; n=%lld gives %d",
                     (long long)in->n, pesq_num_frames(p.n));
     if (!workspace || workspace_bytes < p.total)
-        return fail(FSEM_E_WORKSPACE, "fsem_pesq_score_f32: workspace %zu < %zu bytes", workspace_bytes, p.total);
+        return fail(FSEM_E_WORKSPACE, "fsem_pesq_score: workspace %zu < %zu bytes", workspace_bytes, p.total);
     cudaStream_t stream = static_cast<cudaStream_t>(stream_v);
     char* ws = static_cast<char*>(workspace);
     float* z = reinterpret_cast<float*>(ws + p.off_z);
@@ -447,23 +484,8 @@ extern "C" int fsem_pesq_score(fsem_pesq_ctx_t* ctx, const fsem_batch_t* in, int
     if (p.resample) {   // resample-on-ingest to 16 kHz (base.py:19-20), then the pipeline runs on the workspace copy
         float* y = reinterpret_cast<float*>(ws + p.off_rs);
         int32_t* rslen = reinterpret_cast<int32_t*>(ws + p.off_rslen);
-        const int64_t bps = ceil_div(p.n, 256);
-        if (bps * 2 * in->batch >= (int64_t(1) << 31))
-            return fail(FSEM_E_INVALID, "fsem_pesq_score_f32: batch x samples too large for one launch; split the batch");
-        { ProfScope prof_(K_PESQ_RESAMPLE, stream);
-          dispatch_dtype(dtype, [&](auto tag) {
-              using T = decltype(tag);
-              stoi_resample_kernel<T><<<(unsigned)(bps * 2 * in->batch), 256, 0, stream>>>(
-                  reinterpret_cast<const T*>(in->clean), reinterpret_cast<const T*>(in->deg), in->lengths, in->batch, in->n,
-                  in->stride, ctx->d_rs_taps, ctx->rs_orig, ctx->rs_neu, ctx->rs_width, ctx->rs_ntaps, y, p.rstride, (int)bps);
-              return FSEM_OK;
-          }); }
-        FSEM_LAUNCHED();
-        if (in->lengths) {
-            resampled_lengths_kernel<<<(unsigned)ceil_div(in->batch, 256), 256, 0, stream>>>(
-                in->lengths, in->batch, in->n, ctx->rs_orig, ctx->rs_neu, rslen);
-            FSEM_LAUNCHED();
-        }
+        const int rc = ctx->rs.launch("fsem_pesq_score", K_PESQ_RESAMPLE, in, dtype, y, p.rstride, rslen, stream);
+        if (rc != FSEM_OK) return rc;
         rs_batch = fsem_batch_t{y, y + in->batch * p.rstride, in->lengths ? rslen : nullptr, in->batch, p.n, p.rstride};
         in = &rs_batch;
         dtype = FSEM_DTYPE_F32;                                   // the rest of the chain reads the resampled fp32 rows
@@ -563,14 +585,15 @@ extern "C" int fsem_pesq_debug_taps(fsem_pesq_ctx_t* ctx, int64_t batch, int64_t
 // ================================================================================================
 struct fsem_stoi_ctx {
     DeviceInfo dev;
-    int orig = 1, neu = 1, width = 0, ntaps = 0;
-    float* d_taps = nullptr;
+    Resampler rs;               // input -> 10 kHz; its rates feed the frame kernels even when they are equal
     bool fast85 = false;        // taps fit the specialised 8:5 kernel
     Resample85Taps taps85;
     StoiTables* d_tab = nullptr;
     float clip = 0.f, dyn_range = 40.f;
     int tob_ctas_per_sm = 2;
     HostPipe pipe;
+
+    ~fsem_stoi_ctx() { if (d_tab) cudaFree(d_tab); }
 };
 
 namespace {
@@ -586,8 +609,8 @@ StoiPlan stoi_plan(const fsem_stoi_ctx* ctx, int64_t batch, int64_t n) {
     StoiPlan p{};
     p.batch = batch;
     p.n = n;
-    p.resample = ctx->orig != ctx->neu;
-    p.lmax = stoi_resampled_len(n, ctx->orig, ctx->neu);
+    p.resample = ctx->rs.orig != ctx->rs.neu;
+    p.lmax = stoi_resampled_len(n, ctx->rs.orig, ctx->rs.neu);
     p.ystride = round_up(p.lmax > 0 ? p.lmax : 1, 4);
     p.t0max = stoi_num_frames(p.lmax);
     if (p.t0max < 1) p.t0max = 1;
@@ -620,8 +643,9 @@ extern "C" int fsem_stoi_create(fsem_stoi_ctx_t** out, const fsem_stoi_design_t*
     if (!out || !d) return fail(FSEM_E_INVALID, "fsem_stoi_create: null argument");
     *out = nullptr;
     if (d->orig <= 0 || d->neu <= 0) return fail(FSEM_E_INVALID, "fsem_stoi_create: bad rates");
-    if (d->orig != d->neu && (!d->taps || d->ntaps != 2 * d->width + d->orig || d->width < 0))
-        return fail(FSEM_E_INVALID, "fsem_stoi_create: bad resampling kernel (ntaps must be 2*width+orig)");
+    int rc = d->orig != d->neu ? Resampler::check("fsem_stoi_create", d->orig, d->neu, d->width, d->ntaps, d->taps)
+                               : FSEM_OK;
+    if (rc != FSEM_OK) return rc;
     for (int b = 0; b < FSEM_STOI_NBANDS; ++b)
         if (d->band_lo[b] < 0 || d->band_hi[b] < d->band_lo[b] || d->band_hi[b] > 256)
             return fail(FSEM_E_INVALID, "fsem_stoi_create: band %d outside bins 0..255", b);
@@ -630,29 +654,18 @@ extern "C" int fsem_stoi_create(fsem_stoi_ctx_t** out, const fsem_stoi_design_t*
     for (int b = 0; b + 1 < FSEM_STOI_NBANDS; ++b)
         if (d->band_hi[b] != d->band_lo[b + 1] || d->band_hi[b] - d->band_lo[b] > 48)
             return fail(FSEM_E_INVALID, "fsem_stoi_create: third-octave bands must be contiguous and at most 48 bins wide");
-    fsem_stoi_ctx* ctx = new (std::nothrow) fsem_stoi_ctx();
+    std::unique_ptr<fsem_stoi_ctx> ctx(new (std::nothrow) fsem_stoi_ctx());
     if (!ctx) return fail(FSEM_E_INVALID, "out of host memory");
-    int rc = query_device(ctx->dev);
-    if (rc != FSEM_OK) { delete ctx; return rc; }
-    ctx->orig = d->orig; ctx->neu = d->neu; ctx->width = d->width; ctx->ntaps = d->ntaps;
+    if ((rc = query_device(ctx->dev)) != FSEM_OK) return rc;
     ctx->clip = d->clip; ctx->dyn_range = d->dyn_range;
     StoiTables h{};
     memcpy(h.window, d->window, sizeof(h.window));
     for (int b = 0; b < FSEM_STOI_NBANDS; ++b) { h.band_lo[b] = d->band_lo[b]; h.band_hi[b] = d->band_hi[b]; }
     h.clip = d->clip; h.dyn_range = d->dyn_range;
-    cudaError_t e = cudaMalloc(&ctx->d_tab, sizeof(StoiTables));
-    if (e == cudaSuccess) e = cudaMemcpy(ctx->d_tab, &h, sizeof(h), cudaMemcpyHostToDevice);
-    if (e == cudaSuccess && d->orig != d->neu) {
-        e = cudaMalloc(&ctx->d_taps, sizeof(float) * d->neu * d->ntaps);
-        if (e == cudaSuccess)
-            e = cudaMemcpy(ctx->d_taps, d->taps, sizeof(float) * d->neu * d->ntaps, cudaMemcpyHostToDevice);
-    }
-    if (e != cudaSuccess) {
-        if (ctx->d_tab) cudaFree(ctx->d_tab);
-        if (ctx->d_taps) cudaFree(ctx->d_taps);
-        delete ctx;
-        return fail(FSEM_E_CUDA, "fsem_stoi_create: %s", cudaGetErrorString(e));
-    }
+    FSEM_CUDA(cudaMalloc(&ctx->d_tab, sizeof(StoiTables)));
+    FSEM_CUDA(cudaMemcpy(ctx->d_tab, &h, sizeof(h), cudaMemcpyHostToDevice));
+    ctx->rs.orig = d->orig; ctx->rs.neu = d->neu;
+    if (d->orig != d->neu && (rc = ctx->rs.upload(d->orig, d->neu, d->width, d->ntaps, d->taps)) != FSEM_OK) return rc;
     if (d->orig == 8 && d->neu == 5 && d->width == 10 && d->ntaps == 28) {
         ctx->fast85 = true;
         for (int p = 0; p < 5; ++p)
@@ -664,15 +677,11 @@ extern "C" int fsem_stoi_create(fsem_stoi_ctx_t** out, const fsem_stoi_design_t*
     int occ = 0;
     if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, stoi_tob_kernel<true>, kTobWarps * 32, 0) == cudaSuccess && occ > 0)
         ctx->tob_ctas_per_sm = occ;
-    *out = ctx;
+    *out = ctx.release();
     return FSEM_OK;
 }
 
 extern "C" int fsem_stoi_destroy(fsem_stoi_ctx_t* ctx) {
-    if (!ctx) return FSEM_OK;
-    ctx->pipe.destroy();
-    if (ctx->d_tab) cudaFree(ctx->d_tab);
-    if (ctx->d_taps) cudaFree(ctx->d_taps);
     delete ctx;
     return FSEM_OK;
 }
@@ -694,20 +703,15 @@ extern "C" int fsem_stoi_score_f32(fsem_stoi_ctx_t* ctx, const fsem_batch_t* in,
 extern "C" int fsem_stoi_score(fsem_stoi_ctx_t* ctx, const fsem_batch_t* in, int dtype, float* stoi_out,
                                float* estoi_out, int32_t* kept_frames_out, int32_t* status_out,
                                void* workspace, size_t workspace_bytes, void* stream_v) {
-    if (!ctx || !in || !stoi_out || !estoi_out) return fail(FSEM_E_INVALID, "fsem_stoi_score_f32: null argument");
+    if (!ctx || !in || !stoi_out || !estoi_out) return fail(FSEM_E_INVALID, "fsem_stoi_score: null argument");
     if (dtype_size(dtype) == 0) return fail(FSEM_E_INVALID, "fsem_stoi_score: unknown dtype %d", dtype);
-    if (in->batch < 0 || in->n < 0 || in->stride < in->n)
-        return fail(FSEM_E_INVALID, "fsem_stoi_score_f32: bad shape batch=%lld n=%lld stride=%lld",
-                    (long long)in->batch, (long long)in->n, (long long)in->stride);
-    if (in->batch == 0) return FSEM_OK;
-    if (in->n == 0) return fail(FSEM_E_INVALID, "fsem_stoi_score_f32: n = 0 (empty signals)");
-    if (!in->clean || !in->deg) return fail(FSEM_E_INVALID, "fsem_stoi_score_f32: null input");
-    if (in->n >= (int64_t(1) << 30)) return fail(FSEM_E_INVALID, "fsem_stoi_score_f32: n too large");
+    if (int rc = check_batch("fsem_stoi_score", in->clean, in->deg, in->batch, in->n, in->stride, 1, kMaxN, false))
+        return rc == kEmptyBatch ? FSEM_OK : rc;
     const StoiPlan p = stoi_plan(ctx, in->batch, in->n);
     if (in->batch * (int64_t)p.t0max >= (int64_t(1) << 31))
-        return fail(FSEM_E_INVALID, "fsem_stoi_score_f32: batch x frames exceeds 2^31; split the batch");
+        return fail(FSEM_E_INVALID, "fsem_stoi_score: batch x frames exceeds 2^31; split the batch");
     if (!workspace || workspace_bytes < p.total)
-        return fail(FSEM_E_WORKSPACE, "fsem_stoi_score_f32: workspace %zu < %zu bytes", workspace_bytes, p.total);
+        return fail(FSEM_E_WORKSPACE, "fsem_stoi_score: workspace %zu < %zu bytes", workspace_bytes, p.total);
     cudaStream_t stream = static_cast<cudaStream_t>(stream_v);
     char* ws = static_cast<char*>(workspace);
     float* y = reinterpret_cast<float*>(ws + p.off_y);
@@ -743,20 +747,11 @@ extern "C" int fsem_stoi_score(fsem_stoi_ctx_t* ctx, const fsem_batch_t* in, int
                           p.hops_max, (int)bps);
                   return FSEM_OK;
               }); }
+            FSEM_LAUNCHED();
         } else {
-            const int64_t bps = ceil_div(p.lmax, 256);
-            if (bps * 2 * in->batch >= (int64_t(1) << 31))
-                return fail(FSEM_E_INVALID, "fsem_stoi_score_f32: batch x samples too large for one launch; split the batch");
-            { ProfScope prof_(K_STOI_RESAMPLE, stream);
-              dispatch_dtype(dtype, [&](auto tag) {
-                  using T = decltype(tag);
-                  stoi_resample_kernel<T><<<(unsigned)(bps * 2 * in->batch), 256, 0, stream>>>(
-                      reinterpret_cast<const T*>(in->clean), reinterpret_cast<const T*>(in->deg), in->lengths, in->batch,
-                      in->n, in->stride, ctx->d_taps, ctx->orig, ctx->neu, ctx->width, ctx->ntaps, y, p.ystride, (int)bps);
-                  return FSEM_OK;
-              }); }
+            const int rc = ctx->rs.launch("fsem_stoi_score", K_STOI_RESAMPLE, in, dtype, y, p.ystride, nullptr, stream);
+            if (rc != FSEM_OK) return rc;
         }
-        FSEM_LAUNCHED();
         c10 = y;
         d10 = y + in->batch * p.ystride;
         sstride = p.ystride;
@@ -780,13 +775,13 @@ extern "C" int fsem_stoi_score(fsem_stoi_ctx_t* ctx, const fsem_batch_t* in, int
         const int64_t warps = in->batch * (int64_t)p.t0max;
         { ProfScope prof_(K_STOI_ENERGY, stream);
           stoi_energy_kernel<<<(unsigned)ceil_div(warps * 32, 256), 256, 0, stream>>>(
-            c10, sstride, in->lengths, in->batch, in->n, ctx->orig, ctx->neu, p.t0max, ctx->d_tab, energy); }
+            c10, sstride, in->lengths, in->batch, in->n, ctx->rs.orig, ctx->rs.neu, p.t0max, ctx->d_tab, energy); }
         FSEM_LAUNCHED();
     }
     {
         { ProfScope prof_(K_STOI_COMPACT, stream);
           stoi_compact_kernel<<<(unsigned)ceil_div(in->batch * 32, 128), 128, 0, stream>>>(
-              energy, in->lengths, in->batch, in->n, ctx->orig, ctx->neu, p.t0max, p.mask_words, ctx->dyn_range,
+              energy, in->lengths, in->batch, in->n, ctx->rs.orig, ctx->rs.neu, p.t0max, p.mask_words, ctx->dyn_range,
               kept_idx, kept_count, mask); }
         FSEM_LAUNCHED();
     }
@@ -855,7 +850,7 @@ extern "C" int fsem_stoi_mask_margin(fsem_stoi_ctx_t* ctx, int64_t batch, int64_
     const float* energy = reinterpret_cast<const float*>(static_cast<const char*>(workspace) + p.off_energy);
     { ProfScope prof_(K_STOI_MARGIN, stream);
       stoi_margin_kernel<<<(unsigned)ceil_div(batch * 32, 128), 128, 0, stream>>>(
-          energy, lengths, batch, n, ctx->orig, ctx->neu, p.t0max, ctx->dyn_range, margin_out); }
+          energy, lengths, batch, n, ctx->rs.orig, ctx->rs.neu, p.t0max, ctx->dyn_range, margin_out); }
     FSEM_LAUNCHED();
     return FSEM_OK;
 }
@@ -903,8 +898,8 @@ int score_host_any(const char* who, fsem_pesq_ctx* pctx, fsem_stoi_ctx* sctx, co
         return fail(FSEM_E_INVALID, "%s: null argument", who);
     const size_t es = dtype_size(dtype);
     if (es == 0) return fail(FSEM_E_INVALID, "%s: unknown dtype %d", who, dtype);
-    if (batch < 0 || n < 0 || stride < n) return fail(FSEM_E_INVALID, "%s: bad shape", who);
-    if (batch == 0) return FSEM_OK;
+    if (int rc = check_batch(who, clean, deg, batch, n, stride, 0, INT64_MAX, false))
+        return rc == kEmptyBatch ? FSEM_OK : rc;
     if (pctx && !lengths && pesq_num_frames(pesq_plan(pctx, 1, n).n) < 20)
         return fail(FSEM_E_TOO_SHORT, "PESQ needs at least 20 frames of 512/256 samples at 16 kHz; n=%lld is too short",
                     (long long)n);
@@ -917,11 +912,10 @@ int score_host_any(const char* who, fsem_pesq_ctx* pctx, fsem_stoi_ctx* sctx, co
     const int64_t per = host_chunk_items(batch, n, es);
     const size_t raw_sig = align256(es * per * rstride);
     const size_t in_bytes = 2 * raw_sig + align256(sizeof(int32_t) * per);
-    const size_t conv_sig = 0;
     const size_t ws_pesq = pctx ? align256(fsem_pesq_workspace_bytes(pctx, per, n)) : 0;
     const size_t ws_stoi = sctx ? align256(fsem_stoi_workspace_bytes(sctx, per, n)) : 0;
     const size_t col = align256(sizeof(float) * batch);
-    rc = P.reserve(in_bytes, 2 * conv_sig + ws_pesq + ws_stoi, 6 * col);
+    rc = P.reserve(in_bytes, ws_pesq + ws_stoi, 6 * col);
     if (rc != FSEM_OK) return rc;
     char* const ob = static_cast<char*>(P.out);
     char* const wsb = static_cast<char*>(P.ws);
@@ -957,17 +951,16 @@ int score_host_any(const char* who, fsem_pesq_ctx* pctx, fsem_stoi_ctx* sctx, co
                                           reinterpret_cast<float*>(ob + 2 * col) + i0,
                                           reinterpret_cast<float*>(ob + 3 * col) + i0,
                                           reinterpret_cast<int32_t*>(ob + 4 * col) + i0,
-                                          reinterpret_cast<int32_t*>(ob + 5 * col) + i0, wsb + 2 * conv_sig, ws_pesq,
-                                          wsb + 2 * conv_sig + ws_pesq, ws_stoi, P.compute);
+                                          reinterpret_cast<int32_t*>(ob + 5 * col) + i0, wsb, ws_pesq, wsb + ws_pesq,
+                                          ws_stoi, P.compute);
         else if (rc == FSEM_OK && pctx)
             rc = fsem_pesq_score(pctx, &dev, dtype, reinterpret_cast<float*>(ob) + i0,
-                                 reinterpret_cast<int32_t*>(ob + col) + i0, wsb + 2 * conv_sig, ws_pesq, P.compute);
+                                 reinterpret_cast<int32_t*>(ob + col) + i0, wsb, ws_pesq, P.compute);
         else if (rc == FSEM_OK && sctx)
             rc = fsem_stoi_score(sctx, &dev, dtype, reinterpret_cast<float*>(ob + 2 * col) + i0,
                                      reinterpret_cast<float*>(ob + 3 * col) + i0,
                                      reinterpret_cast<int32_t*>(ob + 4 * col) + i0,
-                                     reinterpret_cast<int32_t*>(ob + 5 * col) + i0, wsb + 2 * conv_sig + ws_pesq, ws_stoi,
-                                     P.compute);
+                                     reinterpret_cast<int32_t*>(ob + 5 * col) + i0, wsb + ws_pesq, ws_stoi, P.compute);
         if (rc != FSEM_OK) return rc;
         FSEM_CUDA(cudaEventRecord(P.done[slot], P.compute));
     }
@@ -1003,7 +996,9 @@ extern "C" int fsem_ingest_f32(const void* src, int dtype, int64_t rows, int64_t
                                int64_t dst_stride, void* stream) {
     if (!src || !dst) return fail(FSEM_E_INVALID, "fsem_ingest_f32: null argument");
     if (dtype_size(dtype) == 0) return fail(FSEM_E_INVALID, "fsem_ingest_f32: unknown dtype %d", dtype);
-    if (rows < 0 || n < 0 || src_stride < n || dst_stride < n) return fail(FSEM_E_INVALID, "fsem_ingest_f32: bad shape");
+    if (dst_stride < n) return fail(FSEM_E_INVALID, "fsem_ingest_f32: dst_stride %lld < n", (long long)dst_stride);
+    if (int rc = check_batch("fsem_ingest_f32", src, dst, rows, n, src_stride, 0, INT64_MAX, false))
+        return rc == kEmptyBatch ? FSEM_OK : rc;
     return launch_ingest(src, dtype, rows, n, src_stride, dst, dst_stride, static_cast<cudaStream_t>(stream));
 }
 
@@ -1044,34 +1039,22 @@ extern "C" int fsem_pesq_stoi_score_host_f32(fsem_pesq_ctx_t* pctx, fsem_stoi_ct
 // general polyphase kernel behind a small context that owns the device copy of the taps.  PESQ and STOI run the
 // same kernel inside their own chains; LSD and SDR call this first.
 // ================================================================================================
-struct fsem_resampler {
-    int orig = 1, neu = 1, width = 0, ntaps = 0;
-    float* d_taps = nullptr;
-};
+struct fsem_resampler : Resampler {};
 
 extern "C" int fsem_resampler_create(fsem_resampler_t** out, int32_t orig, int32_t neu, int32_t width, int32_t ntaps,
                                      const float* taps) {
     if (!out) return fail(FSEM_E_INVALID, "fsem_resampler_create: null argument");
     *out = nullptr;
-    if (orig <= 0 || neu <= 0 || width < 0 || !taps || ntaps != 2 * width + orig)
-        return fail(FSEM_E_INVALID, "fsem_resampler_create: bad resampling kernel (ntaps must be 2*width+orig)");
-    fsem_resampler* r = new (std::nothrow) fsem_resampler();
+    int rc = Resampler::check("fsem_resampler_create", orig, neu, width, ntaps, taps);
+    if (rc != FSEM_OK) return rc;
+    std::unique_ptr<fsem_resampler> r(new (std::nothrow) fsem_resampler());
     if (!r) return fail(FSEM_E_INVALID, "out of host memory");
-    r->orig = orig; r->neu = neu; r->width = width; r->ntaps = ntaps;
-    cudaError_t e = cudaMalloc(&r->d_taps, sizeof(float) * neu * ntaps);
-    if (e == cudaSuccess) e = cudaMemcpy(r->d_taps, taps, sizeof(float) * neu * ntaps, cudaMemcpyHostToDevice);
-    if (e != cudaSuccess) {
-        if (r->d_taps) cudaFree(r->d_taps);
-        delete r;
-        return fail(FSEM_E_CUDA, "fsem_resampler_create: %s", cudaGetErrorString(e));
-    }
-    *out = r;
+    if ((rc = r->upload(orig, neu, width, ntaps, taps)) != FSEM_OK) return rc;
+    *out = r.release();
     return FSEM_OK;
 }
 
 extern "C" int fsem_resampler_destroy(fsem_resampler_t* r) {
-    if (!r) return FSEM_OK;
-    if (r->d_taps) cudaFree(r->d_taps);
     delete r;
     return FSEM_OK;
 }
@@ -1084,29 +1067,14 @@ extern "C" int64_t fsem_resampled_len(const fsem_resampler_t* r, int64_t n) {
 extern "C" int fsem_resample_f32(fsem_resampler_t* r, const fsem_batch_t* in, float* out, int64_t out_stride,
                                  int32_t* lengths_out, void* stream_v) {
     if (!r || !in || !out) return fail(FSEM_E_INVALID, "fsem_resample_f32: null argument");
-    if (in->batch < 0 || in->n <= 0 || in->stride < in->n || in->n >= (int64_t(1) << 30))
-        return fail(FSEM_E_INVALID, "fsem_resample_f32: bad shape");
-    if (in->batch == 0) return FSEM_OK;
-    if (!in->clean || !in->deg) return fail(FSEM_E_INVALID, "fsem_resample_f32: null input");
+    if (int rc = check_batch("fsem_resample_f32", in->clean, in->deg, in->batch, in->n, in->stride, 1, kMaxN, true))
+        return rc == kEmptyBatch ? FSEM_OK : rc;
     const int64_t L = stoi_resampled_len(in->n, r->orig, r->neu);
     if (out_stride < L) return fail(FSEM_E_INVALID, "fsem_resample_f32: out_stride %lld < resampled length %lld",
                                     (long long)out_stride, (long long)L);
     if (in->lengths && !lengths_out) return fail(FSEM_E_INVALID, "fsem_resample_f32: lengths given but lengths_out is null");
-    cudaStream_t stream = static_cast<cudaStream_t>(stream_v);
-    const int64_t bps = ceil_div(L, 256);
-    if (bps * 2 * in->batch >= (int64_t(1) << 31))
-        return fail(FSEM_E_INVALID, "fsem_resample_f32: batch x samples too large for one launch; split the batch");
-    { ProfScope prof_(K_PESQ_RESAMPLE, stream);
-      stoi_resample_kernel<<<(unsigned)(bps * 2 * in->batch), 256, 0, stream>>>(
-          in->clean, in->deg, in->lengths, in->batch, in->n, in->stride, r->d_taps, r->orig, r->neu, r->width,
-          r->ntaps, out, out_stride, (int)bps); }
-    FSEM_LAUNCHED();
-    if (in->lengths) {
-        resampled_lengths_kernel<<<(unsigned)ceil_div(in->batch, 256), 256, 0, stream>>>(
-            in->lengths, in->batch, in->n, r->orig, r->neu, lengths_out);
-        FSEM_LAUNCHED();
-    }
-    return FSEM_OK;
+    return r->launch("fsem_resample_f32", K_PESQ_RESAMPLE, in, FSEM_DTYPE_F32, out, out_stride, lengths_out,
+                     static_cast<cudaStream_t>(stream_v));
 }
 
 // ================================================================================================
@@ -1116,6 +1084,8 @@ struct fsem_lsd_ctx {
     DeviceInfo dev;
     float* d_hann = nullptr;
     int ctas_per_sm = 2;
+
+    ~fsem_lsd_ctx() { if (d_hann) cudaFree(d_hann); }
 };
 
 namespace {
@@ -1134,27 +1104,20 @@ LsdPlan lsd_plan(int64_t batch, int64_t n) {
 extern "C" int fsem_lsd_create(fsem_lsd_ctx_t** out, const float* hann512) {
     if (!out || !hann512) return fail(FSEM_E_INVALID, "fsem_lsd_create: null argument");
     *out = nullptr;
-    fsem_lsd_ctx* ctx = new (std::nothrow) fsem_lsd_ctx();
+    std::unique_ptr<fsem_lsd_ctx> ctx(new (std::nothrow) fsem_lsd_ctx());
     if (!ctx) return fail(FSEM_E_INVALID, "out of host memory");
-    int rc = query_device(ctx->dev);
-    if (rc != FSEM_OK) { delete ctx; return rc; }
-    cudaError_t e = cudaMalloc(&ctx->d_hann, sizeof(float) * 512);
-    if (e == cudaSuccess) e = cudaMemcpy(ctx->d_hann, hann512, sizeof(float) * 512, cudaMemcpyHostToDevice);
-    if (e != cudaSuccess) {
-        if (ctx->d_hann) cudaFree(ctx->d_hann);
-        delete ctx;
-        return fail(FSEM_E_CUDA, "fsem_lsd_create: %s", cudaGetErrorString(e));
-    }
+    const int rc = query_device(ctx->dev);
+    if (rc != FSEM_OK) return rc;
+    FSEM_CUDA(cudaMalloc(&ctx->d_hann, sizeof(float) * 512));
+    FSEM_CUDA(cudaMemcpy(ctx->d_hann, hann512, sizeof(float) * 512, cudaMemcpyHostToDevice));
     int occ = 0;
     if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, lsd_frames_kernel<true>, kLsdWarps * 32, 0) == cudaSuccess && occ > 0)
         ctx->ctas_per_sm = occ;
-    *out = ctx;
+    *out = ctx.release();
     return FSEM_OK;
 }
 
 extern "C" int fsem_lsd_destroy(fsem_lsd_ctx_t* ctx) {
-    if (!ctx) return FSEM_OK;
-    if (ctx->d_hann) cudaFree(ctx->d_hann);
     delete ctx;
     return FSEM_OK;
 }
@@ -1167,10 +1130,8 @@ extern "C" size_t fsem_lsd_workspace_bytes(const fsem_lsd_ctx_t* ctx, int64_t ba
 extern "C" int fsem_lsd_score_f32(fsem_lsd_ctx_t* ctx, const fsem_batch_t* in, float* lsd_out, void* workspace,
                                   size_t workspace_bytes, void* stream_v) {
     if (!ctx || !in || !lsd_out) return fail(FSEM_E_INVALID, "fsem_lsd_score_f32: null argument");
-    if (in->batch < 0 || in->n <= 0 || in->stride < in->n || in->n >= (int64_t(1) << 30))
-        return fail(FSEM_E_INVALID, "fsem_lsd_score_f32: bad shape");
-    if (in->batch == 0) return FSEM_OK;
-    if (!in->clean || !in->deg) return fail(FSEM_E_INVALID, "fsem_lsd_score_f32: null input");
+    if (int rc = check_batch("fsem_lsd_score_f32", in->clean, in->deg, in->batch, in->n, in->stride, 1, kMaxN, true))
+        return rc == kEmptyBatch ? FSEM_OK : rc;
     const LsdPlan p = lsd_plan(in->batch, in->n);
     if (!workspace || workspace_bytes < p.total)
         return fail(FSEM_E_WORKSPACE, "fsem_lsd_score_f32: workspace %zu < %zu bytes", workspace_bytes, p.total);
@@ -1429,10 +1390,8 @@ extern "C" size_t fsem_sdr_workspace_bytes(int64_t batch, int64_t n) {
 extern "C" int fsem_sdr_score_f32(const fsem_batch_t* in, float* sdr_out, void* workspace, size_t workspace_bytes,
                                   void* stream_v) {
     if (!in || !sdr_out) return fail(FSEM_E_INVALID, "fsem_sdr_score_f32: null argument");
-    if (in->batch < 0 || in->n <= 0 || in->stride < in->n || in->n >= (int64_t(1) << 30))
-        return fail(FSEM_E_INVALID, "fsem_sdr_score_f32: bad shape");
-    if (in->batch == 0) return FSEM_OK;
-    if (!in->clean || !in->deg) return fail(FSEM_E_INVALID, "fsem_sdr_score_f32: null input");
+    if (int rc = check_batch("fsem_sdr_score_f32", in->clean, in->deg, in->batch, in->n, in->stride, 1, kMaxN, true))
+        return rc == kEmptyBatch ? FSEM_OK : rc;
     if (in->batch > 65535) return fail(FSEM_E_INVALID, "fsem_sdr_score_f32: batch > 65535; split the batch");
     const SdrPlan p = sdr_plan(in->batch, in->n);
     if (!workspace || workspace_bytes < p.total)

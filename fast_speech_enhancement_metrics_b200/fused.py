@@ -15,6 +15,7 @@ import warnings
 import torch
 
 from . import _lib
+from .base import check_score, make_batch, score_host, stream_ptr
 from .PESQ import PESQ
 from .STOI import STOI
 
@@ -32,17 +33,14 @@ def score_pesq_stoi_tensors(pesq: PESQ, stoi: STOI, clean: torch.Tensor, deg: to
     pst = torch.empty(b, dtype=torch.int32, device=clean.device)
     kept = torch.empty(b, dtype=torch.int32, device=clean.device)
     sst = torch.empty(b, dtype=torch.int32, device=clean.device)
+    batch, clean, deg = make_batch(clean, deg, lens)
     with torch.cuda.device(clean.device):
-        if deg.stride(0) != clean.stride(0) and b > 1:
-            deg = deg.contiguous(); clean = clean.contiguous()
         wp = pesq._get_workspace(pesq._lib.fsem_pesq_workspace_bytes(pesq._ctx, b, n))
         wsb = stoi._get_workspace(stoi._lib.fsem_stoi_workspace_bytes(stoi._ctx, b, n))
-        batch = _lib.Batch(clean.data_ptr(), deg.data_ptr(), lens.data_ptr() if lens is not None else None,
-                           b, n, clean.stride(0) if b > 1 else max(n, clean.stride(0)))
-        PESQ._check_score(pesq._lib.fsem_pesq_stoi_score(
+        check_score(pesq._lib.fsem_pesq_stoi_score(
             pesq._ctx, stoi._ctx, C.byref(batch), _lib.dtype_code(clean.dtype), scores[0].data_ptr(), pst.data_ptr(), scores[1].data_ptr(),
             scores[2].data_ptr(), kept.data_ptr(), sst.data_ptr(), wp.data_ptr(), wp.numel(), wsb.data_ptr(),
-            wsb.numel(), C.c_void_p(torch.cuda.current_stream(clean.device).cuda_stream)))
+            wsb.numel(), stream_ptr(clean.device)))
     pesq._last_shape = (b, n)
     stoi._last_shape = (b, n)
     stoi._last_lengths = lens
@@ -57,26 +55,13 @@ def score_pesq_stoi(pesq: PESQ, stoi: STOI, clean_speech: torch.Tensor, denoised
         raise Exception("both metrics must be built for the sample rate of the audio")
     clean, deg = pesq.prepare_inputs(clean_speech, denoised_speech)
     assert clean is not None
-    b, n = clean.shape
     if clean.is_cuda:
         # device-resident tensors: one library call for both kernel chains
         scores, pst, kept, _ = score_pesq_stoi_tensors(pesq, stoi, clean, deg, lengths)
         packed = torch.cat([scores, pst.to(torch.float32)[None], kept.to(torch.float32)[None]]).cpu()
         mos, sc, pst, kept = packed[0], packed[1:3], packed[3].to(torch.int32), packed[4].to(torch.int32)
     else:
-        lens = pesq._lengths_tensor(lengths, b, n, "cpu")
-        mos = torch.empty(b, dtype=torch.float32)
-        pst = torch.empty(b, dtype=torch.int32)
-        sc = torch.empty(2, b, dtype=torch.float32)
-        kept = torch.empty(b, dtype=torch.int32)
-        sst = torch.empty(b, dtype=torch.int32)
-        if clean.stride(0) != deg.stride(0) and b > 1:
-            clean, deg = clean.contiguous(), deg.contiguous()
-        with torch.cuda.device(pesq.device):
-            PESQ._check_score(pesq._lib.fsem_score_host(
-                pesq._ctx, stoi._ctx, clean.data_ptr(), deg.data_ptr(), _lib.dtype_code(clean.dtype),
-                lens.data_ptr() if lens is not None else None, b, n, clean.stride(0) if b > 1 else n,
-                mos.data_ptr(), pst.data_ptr(), sc[0].data_ptr(), sc[1].data_ptr(), kept.data_ptr(), sst.data_ptr()))
+        mos, pst, sc, kept, _ = score_host(pesq, stoi, clean, deg, lengths)
     if lengths is not None and bool((pst == _lib.ITEM_TOO_SHORT).any()):
         raise RuntimeError("PESQ needs at least 20 frames of 512/256 samples for every item")
     stoi.last_kept_frames = kept
@@ -133,10 +118,9 @@ class CapturedScorer:
         self.stoi_status = torch.zeros(b, dtype=torch.int32, device=clean.device)
         # the library cuts the batch into `slices` parts (0: its own choice) and owns the graph's workspaces
         self._handle = C.c_void_p()
-        batch = _lib.Batch(clean.data_ptr(), deg.data_ptr(), self.lengths.data_ptr() if self.lengths is not None else None,
-                           b, n, clean.stride(0) if b > 1 else max(n, clean.stride(0)))
+        batch, _, _ = make_batch(clean, deg, self.lengths)      # same pitch (checked above): points at clean / deg
         with torch.cuda.device(self.device):
-            PESQ._check_score(self._lib.fsem_graph_create(
+            check_score(self._lib.fsem_graph_create(
                 C.byref(self._handle), pesq._ctx if pesq is not None else None, stoi._ctx if stoi is not None else None,
                 C.byref(batch), _lib.dtype_code(clean.dtype), self.scores[0].data_ptr(), self.pesq_status.data_ptr(),
                 self.scores[1].data_ptr(), self.scores[2].data_ptr(), self.kept_frames.data_ptr(),
@@ -150,8 +134,7 @@ class CapturedScorer:
         if not getattr(self, "_handle", None):
             raise Exception("CapturedScorer is closed")
         with torch.cuda.device(self.device):
-            _lib.check(self._lib.fsem_graph_launch(
-                self._handle, C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)))
+            _lib.check(self._lib.fsem_graph_launch(self._handle, stream_ptr(self.device)))
         return self.scores, self.pesq_status, self.kept_frames, self.stoi_status
 
     def __call__(self) -> list[dict[str, float]]:

@@ -25,7 +25,10 @@
  *     points include the host<->device copies and return after the scores are in host memory.
  *   - a context is bound to the CUDA device that was current when it was created and may
  *     be used from one host thread at a time.
- *   - there is no CPU fallback: without a CUDA device every entry point fails with FSEM_E_CUDA.
+ *   - arguments (designs, batch shapes, pointers) are checked before the first CUDA call, so a malformed
+ *     argument gives FSEM_E_INVALID with or without a GPU.
+ *   - there is no CPU fallback: without a CUDA device every call that gets past its argument checks fails
+ *     with FSEM_E_CUDA.
  */
 #ifndef FSEM_H_
 #define FSEM_H_
